@@ -4,6 +4,14 @@ same workload: batch x heads shards with no data-path collective, so scaling is 
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this library
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference's CPU path
+    python bench.py ... --dump-outputs DIR                         # + what the last timed step computed
+
+--steps K is the number of timed steps of every timed pass.  --dump-outputs writes o, dq, dk, dv of the last
+headline step (rank 0) as DIR/{o,dq,dk,dv}.npy, float32 of shape (4, 8, 1024, 64): every (batch, head) at the
+same 1024 sequence positions, drawn with a fixed seed (DUMP_ROWS).  The inputs are seeded too, so two builds
+run with the same arguments can be compared output for output.  o, dk and dv repeat bit for bit from run to run;
+dq is summed over key tiles by fp32 reduce-adds from many CTAs in no fixed order, so its final bf16 rounding can
+land one step apart (4.9e-4 at most, on values up to 2.6, between two runs on a B200 at 1000 W).
 
 One JSON line on stdout (rank 0).  Keys follow the driver contract; in short:
   value        whole-job TFLOP/s, inputs resident in HBM, timed with CUDA events per step
@@ -41,6 +49,7 @@ STEP_FLOPS = FWD_FLOPS + BWD_FLOPS               # 2.405e11
 METRIC = "fwd+bwd TFLOP/s at (4,8,4096,64) bf16 causal"
 C5 = (8, 16, 16384, 128)
 C5_FLOPS = 3.5 * 4 * C5[0] * C5[1] * C5[2] * C5[2] * C5[3] / 2      # 3.079e13
+DUMP_ROWS = 1024                                 # sequence positions kept by --dump-outputs (32 MiB in all)
 
 
 def load_peaks():
@@ -117,8 +126,7 @@ class ClockSampler:
 # ---------------------------------------------------------------------------------------------------
 # the reference arm: the reference's own CPU path on the host cores
 # ---------------------------------------------------------------------------------------------------
-REF_CANDIDATES = ("/root/reference/flash_cosine_sim_attention/flash_cosine_sim_attention.py",
-                  os.path.join(ROOT, "baseline", "_ref", "flash_cosine_sim_attention", "flash_cosine_sim_attention.py"))
+REF_CANDIDATES = (os.path.join(ROOT, "baseline", "_ref", "flash_cosine_sim_attention", "flash_cosine_sim_attention.py"),)
 
 
 def load_reference_plain():
@@ -227,6 +235,20 @@ def bind_to_gpu_numa_node(torch, index):
         return {"node": None, "note": f"not bound ({type(e).__name__})"}
 
 
+def dump_outputs(out_dir, outs):
+    """Write o, dq, dk, dv of one step as float32 DIR/<name>.npy: every (batch, head) at DUMP_ROWS sequence positions
+    drawn with a fixed seed (the full tensors would be 128 MiB).  Returns a description for the JSON line."""
+    import numpy as np
+    import torch
+    rows = np.sort(np.random.default_rng(0).choice(N, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(outs[0].device)
+    names = ("o", "dq", "dk", "dv")
+    for name, t in zip(names, outs):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().index_select(2, idx).float().cpu().numpy())
+    return {"dir": out_dir, "files": [n + ".npy" for n in names], "dtype": "float32",
+            "shape": [B, H, DUMP_ROWS, D], "sample": f"{DUMP_ROWS} of {N} sequence positions, numpy seed 0"}
+
+
 # ---------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -236,9 +258,17 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c5", action="store_true", help="skip the config-5 (8,16,16384,128) sharded measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded sample of o, dq, dk, dv of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl b200")
         return run_reference_arm(args)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -320,10 +350,16 @@ def main():
         for i in range(K):
             flush.zero_()
             ev[i][0].record()
-            step(q, k, v, do)
+            outs = step(q, k, v, do)
             ev[i][1].record()
+            if i < K - 1:
+                # freed at once, as in the warm-up: outputs held into the next step would make the caching
+                # allocator grow (cudaMalloc) inside the timed region
+                del outs
         host_enqueue_us = (time.perf_counter() - host_t0) / K * 1e6      # host time to ENQUEUE one step (no sync inside)
         barrier()
+    dumped = dump_outputs(args.dump_outputs, outs) if args.dump_outputs and rank == 0 else None
+    del outs
     launches_per_step = (debug() - launches0) // (K + 2)
     launches = launches_per_step * K
     step_ms = [a.elapsed_time(b) for a, b in ev]
@@ -424,7 +460,7 @@ def main():
         for _ in range(2):
             c5_step()
         barrier()
-        KC = max(3, min(K, 5))
+        KC = K
         cev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(KC)]
         for i in range(KC):
             cev[i][0].record()
@@ -515,6 +551,8 @@ def main():
         }
         if c5 is not None:
             line["c5"] = c5
+        if dumped is not None:
+            line["dumped_outputs"] = dumped
         if world == 1 and not args.no_cpu_baseline:
             fn, kind, src = load_reference_plain()
             cores = host_threads(torch, fn)                           # calibrates the thread count (also the warm-up)

@@ -1,13 +1,14 @@
 """Pins the oracle to the UNMODIFIED reference and writes the golden vectors.
 
-Run in the build container (needs /root/reference; it cannot run on the GPU box):
-    python oracle/make_golden.py
+Needs a checkout of the reference project (no GPU, no compiled extension):
+    python oracle/make_golden.py PATH/TO/flash-cosine-sim-attention
 
 For each case it (1) loads the reference's flash_cosine_sim_attention.py by path (the package
 import itself fails without the compiled extension, reference __init__.py:1), (2) runs
 `plain_cosine_sim_attention` in float64 with autograd on seeded inputs, (3) asserts that
 oracle/cosine_sim_attention_oracle.py reproduces the outputs and all gradients to 1e-9, and
-(4) stores inputs + reference outputs in tests/golden/<case>.npz.
+(4) stores inputs + reference outputs in tests/golden/<case>.npz.  Shapes are kept small enough that
+every file stays under 1 MB.
 TEST INFRASTRUCTURE ONLY.
 """
 import contextlib
@@ -24,12 +25,12 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 from oracle import cosine_sim_attention_oracle as oracle  # noqa: E402
 
-REF_PY = "/root/reference/flash_cosine_sim_attention/flash_cosine_sim_attention.py"
+REF_PY = os.path.join("flash_cosine_sim_attention", "flash_cosine_sim_attention.py")     # inside the reference
 
 # name -> (q shape, k/v shape, kwargs, has_mask)
 CASES = {
     "c1_noncausal_f32": dict(q=(1, 2, 128, 64), kv=(1, 2, 128, 64), kw=dict()),
-    "causal_square": dict(q=(2, 3, 96, 64), kv=(2, 3, 96, 64), kw=dict(causal=True)),
+    "causal_square": dict(q=(2, 2, 96, 64), kv=(2, 2, 96, 64), kw=dict(causal=True)),
     "causal_cross_40_72": dict(q=(1, 2, 40, 64), kv=(1, 2, 72, 64), kw=dict(causal=True)),
     "causal_cross_72_40": dict(q=(1, 2, 72, 64), kv=(1, 2, 40, 64), kw=dict(causal=True, scale=4)),
     "mask_single_head_kv_groups2": dict(q=(2, 4, 50, 64), kv=(2, 70, 64), kw=dict(groups=2), mask=True),
@@ -37,14 +38,14 @@ CASES = {
     "d128_causal_scale10": dict(q=(1, 2, 64, 128), kv=(1, 2, 64, 128), kw=dict(causal=True, scale=10)),
     "no_l2norm": dict(q=(1, 2, 48, 64), kv=(1, 2, 48, 64), kw=dict(l2norm_qk=False, scale=1), small=True),
     # attn_bias (reference tests/test.py:58-61): per head, and with a batch dimension on merged batch-heads
-    "bias_heads_causal": dict(q=(2, 3, 80, 64), kv=(2, 3, 80, 64), kw=dict(causal=True), bias=(3, 80, 80)),
+    "bias_heads_causal": dict(q=(2, 2, 80, 64), kv=(2, 2, 80, 64), kw=dict(causal=True), bias=(2, 80, 80)),
     "bias_heads_mask_cross": dict(q=(2, 2, 40, 64), kv=(2, 2, 72, 64), kw=dict(), mask=True, bias=(2, 40, 72)),
     "bias_batch_dim_merged": dict(q=(4, 56, 64), kv=(4, 56, 64), kw=dict(attn_bias_batch_dim=True), bias=(4, 56, 56)),
 }
 
 
-def load_reference():
-    spec = importlib.util.spec_from_file_location("ref_fcsa", REF_PY)
+def load_reference(ref_root):
+    spec = importlib.util.spec_from_file_location("ref_fcsa", os.path.join(ref_root, REF_PY))
     mod = importlib.util.module_from_spec(spec)
     with contextlib.redirect_stdout(io.StringIO()):   # it prints a "not compiled" hint
         spec.loader.exec_module(mod)
@@ -52,7 +53,9 @@ def load_reference():
 
 
 def main():
-    ref = load_reference()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python oracle/make_golden.py PATH/TO/flash-cosine-sim-attention")
+    ref = load_reference(sys.argv[1])
     out_dir = os.path.join(ROOT, "tests", "golden")
     os.makedirs(out_dir, exist_ok=True)
     for idx, (name, c) in enumerate(CASES.items()):

@@ -1,5 +1,5 @@
-import time, torch, sys
-sys.path.insert(0, '/root/repo')
+import os, time, torch, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from flash_cosine_sim_attention_b200 import flash_cosine_sim_attention
 dev='cuda'
 for shape in [(4,8,4096,64),(1,8,512,64)]:
